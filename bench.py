@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
     python bench.py --impl reference --steps K --warmup W    # reference algorithm on the host cores (oracle port)
+    python bench.py --steps K --dump-outputs DIR             # also write the outputs of the last timed step (.npy)
 
 One "step" = one call of the Dreamer-V3 update (`train()`, reference dreamer_v3.py:48-357) on one per-rank
 replay batch of the BASELINE config: size S, B=16, T=64, 64x64x3 uint8 observations, horizon 15, discrete A=2.
@@ -122,6 +123,31 @@ def synthetic_batch(cfg, adim, seed, device=None, pinned=False):
     if device is not None:
         d = {k: v.to(device) for k, v in d.items()}
     return d
+
+
+DUMP_CAP = 1 << 21      # elements per dumped array; a larger parameter group is dumped as a fixed, seeded sample
+
+
+def dump_outputs(eng, directory):
+    """Writes what a caller of train() holds after the step: the 13 logged metrics (in METRIC_ORDER), the Moments
+    (low, high) and the four parameter groups, as float32 `.npy` files (at most 8 MB per group)."""
+    import numpy as np
+    import torch
+
+    from sheeprl_b200.algos.dreamer_v3.dreamer_v3 import METRIC_ORDER
+
+    md = eng.metrics_dict()
+    out = {"metrics": torch.stack([md[k] for k in METRIC_ORDER]), "moments": eng.moments_state}
+    for name, group in (("world_model", eng.wm), ("actor", eng.actor), ("critic", eng.critic), ("target_critic", eng.target)):
+        flat = group.flat
+        if flat.numel() > DUMP_CAP:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randint(0, flat.numel(), (DUMP_CAP,), generator=g).sort().values
+            flat = flat[idx.to(flat.device)]
+        out[name] = flat
+    os.makedirs(directory, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -284,6 +310,8 @@ def run_b200(args):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     # ---- timed region 2: `e2e`: the same public call with the batch in pinned HOST memory (H2D inside train()) and
     # a device->host read of the step's 13 metrics
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -587,7 +615,11 @@ def main():
     ap.add_argument("--no-overlap-allreduce", action="store_true", help="one all-reduce of the whole world-model gradient "
                     "before the optimizer instead of three overlapped buckets (the default when the persistent scan runs)")
     ap.add_argument("--overlap-allreduce", action="store_true", help="force the three overlapped bucket reductions")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of `value`, write what the last of them computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.batch is None:
         args.batch = 16 if args.size == "S" else 64
     if args.size != "S" and "--cpu-baseline" not in sys.argv:

@@ -1,7 +1,7 @@
 """Buffer checkpoints (SURVEY §8f-2 / f-3): the device rings pickle like the reference's buffer objects
-(`state["rb"] = rb`, utils/callback.py:37-41), `CheckpointCallback` mirrors the reference's truncated fix-up, and —
-where the reference tree is present — buffers convert to / from the reference's own classes with identical
-subsequent samples."""
+(`state["rb"] = rb`, utils/callback.py:37-41), `CheckpointCallback` mirrors the reference's truncated fix-up, and
+buffers convert to / from the reference's own classes (objects recorded from the executed reference,
+tests/golden/buffer_objects.pt) with identical subsequent samples."""
 import io
 import os
 
@@ -9,11 +9,13 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_harness
 from oracle.ops_emul import EmulOps
 from sheeprl_b200.data import buffers as RB
 from sheeprl_b200.utils.callback import CheckpointCallback, load_replay_buffer
 from tests.buffer_scenarios import seed_rngs, synth_rows
+
+
+KINDS = ("uniform", "sequential", "env_independent")
 
 
 def _rows(length, n_envs, seed):
@@ -52,7 +54,7 @@ def _same_samples(a, b, kw):
         assert sa[k].dtype == sb[k].dtype and np.array_equal(sa[k], sb[k]), k
 
 
-@pytest.mark.parametrize("kind", ["uniform", "sequential", "env_independent"])
+@pytest.mark.parametrize("kind", KINDS)
 def test_pickle_round_trip_continues_identically(kind):
     a, kw = _make(kind)
     bio = io.BytesIO()
@@ -96,28 +98,44 @@ def test_checkpoint_callback_marks_the_last_step_truncated_only_in_the_file(kind
         assert torch.equal(s["truncated"][mask], r["truncated"][mask])
 
 
-needs_reference = pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree absent")
+def _reference_object(rec):
+    """a reference buffer object as recorded by oracle/make_golden_buffer_objects.py: the reference's class name and
+    attributes (what `load_replay_buffer` and `from_reference` see of it), without the reference's code"""
+    attrs = dict(rec["attrs"])
+    st = attrs["_rng"]
+    attrs["_rng"] = np.random.Generator(getattr(np.random, st["bit_generator"])())
+    attrs["_rng"].bit_generator.state = st
+    if isinstance(attrs["_buf"], list):
+        attrs["_buf"] = [_reference_object(r) for r in attrs["_buf"]]
+    obj = type(rec["class"], (), {})()
+    obj.__dict__.update(attrs)
+    return obj
 
 
-@needs_reference
-@pytest.mark.parametrize("kind", ["uniform", "sequential", "env_independent"])
-def test_conversion_to_and_from_the_reference_classes(kind, tmp_path):
-    ref_harness.install()
-    import sheeprl.data.buffers as SB
-
+@pytest.mark.parametrize("kind", KINDS)
+def test_conversion_to_and_from_the_reference_classes(kind, golden_dir):
+    """ours -> reference: the object the reference's class built from this buffer (`to_reference`, through its pickle)
+    holds our rows, write heads and Generator state; reference -> ours: adopting that object (as found in a reference
+    checkpoint) samples exactly what the reference sampled from it."""
+    rec = torch.load(os.path.join(golden_dir, "buffer_objects.pt"), weights_only=False)[kind]
     mine, kw = _make(kind)
-    # ours -> reference object (what a reference run would resume from), also through its pickle and memmap storage
-    for memmap in (False, True):
-        ref = mine.to_reference(memmap=memmap, memmap_dir=tmp_path / f"mm_{kind}_{memmap}" if memmap else None)
-        assert isinstance(ref, getattr(SB, type(mine).__name__))
-        bio = io.BytesIO()
-        torch.save({"rb": ref}, bio)
-        bio.seek(0)
-        ref2 = torch.load(bio, weights_only=False)["rb"]
-        # reference object (as found in a reference checkpoint) -> ours
-        back = load_replay_buffer(ref2, device="cpu", ops=EmulOps())
-        assert type(back) is type(mine) and _heads(back) == _heads(mine)
-        want = ref.sample(**kw)
-        got = back.sample(**kw)
-        for k in want:
-            assert np.array_equal(np.asarray(want[k]), got[k]), (kind, memmap, k)
+    assert kw == rec["sample_kwargs"]
+    ref = _reference_object(rec["object"])
+    assert type(ref).__name__ == type(mine).__name__
+    rings = mine.buffer if isinstance(mine, RB.EnvIndependentReplayBuffer) else [mine]
+    ref_rings = ref._buf if isinstance(mine, RB.EnvIndependentReplayBuffer) else [ref]
+    assert [(r._pos, r._full) for r in ref_rings] == _heads(mine)
+    for r, theirs in zip(rings, ref_rings):
+        assert sorted(theirs._buf) == sorted(r._buf)
+        rows = r.buffer_size if r._full else r._pos                         # rows past the write head hold no data
+        for k, v in theirs._buf.items():
+            ours = r[k].cpu().numpy()
+            assert v.dtype == ours.dtype and v.shape == ours.shape and np.array_equal(v[:rows], ours[:rows]), k
+        assert theirs._rng.bit_generator.state == r._rng.bit_generator.state
+    assert ref._rng.bit_generator.state == mine._rng.bit_generator.state
+    back = load_replay_buffer(ref, device="cpu", ops=EmulOps())
+    assert type(back) is type(mine) and _heads(back) == _heads(mine)
+    got = back.sample(**kw)
+    assert sorted(got) == sorted(rec["sample"])
+    for k, want in rec["sample"].items():
+        assert want.dtype == got[k].dtype and np.array_equal(want, got[k]), (kind, k)

@@ -2,6 +2,8 @@
 No kernel is launched here (no GPU in this container)."""
 import ctypes
 import os
+import subprocess
+import sys
 
 import pytest
 
@@ -30,15 +32,17 @@ def test_library_identity(built):
 
 
 def test_product_path_refuses_to_run_without_gpu():
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from sheeprl_b200.configs import make_dv3_cfg
-    from sheeprl_b200.engine import DV3Engine
-
-    with pytest.raises(L.B200RLError):
-        DV3Engine(make_dv3_cfg("S", per_rank_batch_size=2, per_rank_sequence_length=2), (2,), device="cuda")
+    # in a process that sees no device, so that the check also runs on a machine with a GPU
+    code = ("import pytest\n"
+            "from sheeprl_b200 import lib as L\n"
+            "from sheeprl_b200.configs import make_dv3_cfg\n"
+            "from sheeprl_b200.engine import DV3Engine\n"
+            "with pytest.raises(L.B200RLError):\n"
+            "    DV3Engine(make_dv3_cfg('S', per_rank_batch_size=2, per_rank_sequence_length=2), (2,), device='cuda')\n")
+    root = os.path.dirname(os.path.dirname(os.path.abspath(L.__file__)))
+    r = subprocess.run([sys.executable, "-c", code], cwd=root, capture_output=True, text=True,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stderr[-2000:]
 
 
 def test_product_never_imports_oracle():
